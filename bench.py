@@ -7,7 +7,7 @@ reference's codes, and the fp32 engine's bit-exactness on the same inputs), `par
 roofline), `config2` (NAR B=32 x L=1500), `config3` (256 prompts, strong scaling, every N), `config4` (EnCodec
 encode + decode), `roofline_b1` / `p50_utt_latency_ms` (configs[1]), `cpu_baseline`.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" = one pass of the hot path over one batch of synthetic utterances per GPU:
@@ -53,6 +53,8 @@ def parse():
                     help="BASELINE configs[3]: prompts of the strong-scaling job sharded over the ranks (0 = skip)")
     ap.add_argument("--no-extra", action="store_true",
                     help="skip the sub-objects (parity, parity_mode, config2/3/4, batch-1 latency, cpu_baseline)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the codes the timed path returned in its last step to DIR/codes.npy")
     return ap.parse_args()
 
 
@@ -247,6 +249,22 @@ def cpu_reference_sample(seconds, threads=None, one_thread=True):
 def _golden(name):
     p = os.path.join(ROOT, "tests", "golden", name)
     return torch.load(p, weights_only=False) if os.path.exists(p) else None
+
+
+def dump_codes(out_dir, codes, max_bytes=64 << 20):
+    """codes[b]: int64 [T_b, Q] ids of utterance b -> DIR/codes.npy, float32 [B, max T_b, Q], -1 past each T_b.
+    Above max_bytes only a fixed, seeded sample of the utterances is written (in batch order).  The inputs are seeded
+    and the default decode chain adds its partial sums in fixed order, so two runs with the same arguments write the
+    same file."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    codes = list(codes)
+    row_bytes = max(int(c.shape[0]) for c in codes) * N_Q * 4
+    if len(codes) * row_bytes > max_bytes:
+        keep = torch.randperm(len(codes), generator=torch.Generator().manual_seed(0))[: max_bytes // row_bytes]
+        codes = [codes[i] for i in sorted(keep.tolist())]
+    padded = torch.nn.utils.rnn.pad_sequence(codes, batch_first=True, padding_value=-1)
+    np.save(os.path.join(out_dir, "codes.npy"), padded.cpu().numpy().astype(np.float32))
 
 
 def first_divergence(a, b):
@@ -462,7 +480,7 @@ def main():
         ar_ms = nar_ms = pre_ms = 0.0
         t_wall = time.perf_counter()
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        utt0 = None
+        utt0 = codes = None
         ev0.record()
         for i in range(steps):
             codes = one_step(*batches[i % 2], e2e)
@@ -478,13 +496,15 @@ def main():
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return dict(ms=float(t.item()), wall_ms=wall, launches=eng.kernel_launches() - n0,
-                    ar_ms=ar_ms, nar_ms=nar_ms, prefill_ms=pre_ms, steps=eng.stats.ar_steps, utt0=utt0)
+                    ar_ms=ar_ms, nar_ms=nar_ms, prefill_ms=pre_ms, steps=eng.stats.ar_steps, utt0=utt0, codes=codes)
 
     clocks = Clocks(local)
     if rank == 0:
         clocks.start()
     r = timed(False, a.steps, a.warmup)
     clk = clocks.stop() if rank == 0 else None
+    if a.dump_outputs and rank == 0:
+        dump_codes(a.dump_outputs, r["codes"])
     re = timed(True, a.steps, max(1, min(a.warmup, 1)))
 
     tokens_step = B * frames * N_Q                     # per GPU per step

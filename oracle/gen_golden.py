@@ -2,7 +2,7 @@
 (/root/reference, through oracle/ref_loader.py) on CPU in fp32.  Runs only in the build
 container; the fixtures travel to the GPU box, the reference does not.
 
-    python -m oracle.gen_golden [tiny] [batch] [config0] [big_short] [big_full] [topk]
+    python -m oracle.gen_golden [tiny] [batch] [config0] [big_short] [big_full] [topk] [ref_oracle] [ref_layout]
 
 Every fixture stores: the model config, the weight seed (weights = the reference's default init
 under torch.manual_seed(seed); valle_b200.models.VALLE reproduces them bit-for-bit, checked by
@@ -254,6 +254,57 @@ def gen_switches(ref, only=()):
                                 codes=codes.to(torch.int16), forward=fw))
 
 
+def gen_ref_oracle(ref):
+    """greedy, continual and top-k sampled codes and a training loss of the reference at prefix_mode 0 and 1, on the
+    inputs tests/test_oracle.py feeds the oracle"""
+    import random
+    d, h, l, seed = 256, 4, 2, 0
+    out = {}
+    for pm in (0, 1):
+        m = build_reference(ref, d, h, l, pm, seed)
+        g = torch.Generator().manual_seed(21)
+        x = torch.randint(3, 100, (1, 7), generator=g)
+        y = torch.randint(0, 1024, (1, 15, 8), generator=g)
+        xl = torch.tensor([7], dtype=torch.int32)
+        with torch.no_grad():
+            codes = m.inference(x, xl, y, None, top_k=1)
+            cont = m.continual(x, xl, y)
+            torch.manual_seed(3)
+            sampled = m.inference(x, xl, y, None, top_k=5, temperature=0.9)
+        xx = torch.randint(3, 100, (3, 9), generator=g)
+        xls = torch.tensor([9, 7, 5], dtype=torch.int32)
+        yy = torch.randint(0, 1024, (3, 40, 8), generator=g)
+        yls = torch.tensor([40, 33, 28], dtype=torch.int32)
+        m.rng = random.Random(0)
+        torch.manual_seed(5)
+        with torch.no_grad():
+            (_, _), loss, _ = m(xx, xls, yy, yls)
+        out[f"pm{pm}"] = dict(config=dict(d_model=d, nhead=h, num_layers=l, prefix_mode=pm, num_quantizers=8),
+                              weight_seed=seed, checksums=checksums(m.state_dict()), x=x, y=y,
+                              codes=codes.to(torch.int16), continual=cont.to(torch.int16),
+                              sampled=sampled.to(torch.int16),
+                              forward=dict(x=xx, x_lens=xls, y=yy.to(torch.int16), y_lens=yls,
+                                           loss=torch.as_tensor(float(loss))))
+        print(f"ref_oracle pm={pm}: frames={codes.shape[1]} sampled={sampled.shape[1]} loss={float(loss):.6f}")
+    save("ref_oracle.pt", out)
+
+
+def gen_ref_layout(ref):
+    """the reference's state_dict layout (name -> shape, dtype in order), per-tensor fingerprints and parameter /
+    buffer names: without and with the pre-nets at weight seed 0, and at seed 123 (tests/test_oracle.py,
+    tests/test_boundary.py)"""
+    out = {}
+    for name, prenet, seed in (("prenet0", False, 0), ("prenet1", True, 0), ("seed123", False, 123)):
+        torch.manual_seed(seed)
+        m = ref.VALLE(256, 4, 2, norm_first=True, add_prenet=prenet, prefix_mode=1, share_embedding=True,
+                      nar_scale_factor=1.0, prepend_bos=False, num_quantizers=8)
+        sd = m.state_dict()
+        out[name] = dict(tensors={k: (tuple(v.shape), v.dtype) for k, v in sd.items()}, checksums=checksums(sd),
+                         parameters=[n for n, _ in m.named_parameters()], buffers=[n for n, _ in m.named_buffers()])
+        print(f"ref_layout {name}: {len(sd)} tensors")
+    save("ref_layout.pt", out)
+
+
 def main(argv):
     ref = load_reference()
     what = argv or ["tiny", "batch", "config0", "big_short"]
@@ -274,6 +325,10 @@ def main(argv):
         gen_topk(ref)
     if "big_full" in what:
         gen_big(ref, 47, 225, "big_full")  # BASELINE.json configs[1]: 3 s prompt -> 753 frames
+    if "ref_oracle" in what:
+        gen_ref_oracle(ref)
+    if "ref_layout" in what:
+        gen_ref_layout(ref)
 
 
 if __name__ == "__main__":

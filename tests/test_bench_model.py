@@ -26,6 +26,31 @@ def test_nar_pass_flops_matches_survey_8d():
     assert 0.80 < proj / fb < 0.90
 
 
+def test_dump_codes_pads_ragged_utterances(tmp_path):
+    import numpy as np
+    import torch
+    codes = [torch.arange(24).view(3, 8), torch.full((1, 8), 1024)]
+    bench.dump_codes(str(tmp_path / "out"), codes)
+    got = np.load(tmp_path / "out" / "codes.npy")
+    assert got.dtype == np.float32 and got.shape == (2, 3, 8)
+    assert (got[0] == np.arange(24).reshape(3, 8)).all()
+    assert (got[1, 0] == 1024).all() and (got[1, 1:] == -1).all()
+
+
+def test_dump_codes_samples_utterances_above_the_size_cap(tmp_path):
+    import numpy as np
+    import torch
+    codes = [torch.full((5, 8), b) for b in range(10)]
+    for run in ("a", "b"):
+        bench.dump_codes(str(tmp_path / run), codes, max_bytes=3 * 5 * 8 * 4 + 10)
+    got = np.load(tmp_path / "a" / "codes.npy")
+    assert got.shape == (3, 5, 8) and got.nbytes <= 3 * 5 * 8 * 4
+    rows = got[:, 0, 0].tolist()
+    assert rows == sorted(rows) and len(set(rows)) == 3                 # distinct utterances, in batch order
+    assert all((got[i] == rows[i]).all() for i in range(3))             # whole utterances, not mixed rows
+    assert np.array_equal(got, np.load(tmp_path / "b" / "codes.npy"))   # the same sample every time
+
+
 def test_bench_workload_constants_are_baseline_config1():
     assert (bench.D_MODEL, bench.N_HEAD, bench.N_LAYER, bench.N_Q) == (1024, 16, 12, 8)
     assert (bench.S_TEXT, bench.T_PROMPT) == (47, 225)

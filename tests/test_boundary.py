@@ -32,41 +32,44 @@ def test_valle_package_exports_the_reference_names():
 
 
 def _reference_checkpoint(seed):
-    from oracle.ref_loader import load_reference, reference_available
-    if not reference_available():
-        pytest.skip("/root/reference not mounted (build container only)")
-    ref = load_reference()
-    torch.manual_seed(seed)
-    rm = ref.VALLE(PARAMS["decoder_dim"], PARAMS["nhead"], PARAMS["num_decoder_layers"], norm_first=True,
-                   add_prenet=False, prefix_mode=1, share_embedding=True, nar_scale_factor=1.0, prepend_bos=False,
-                   num_quantizers=8)
-    # the trainer's checkpoint: {"model": state_dict, ...flattened params} (valle/bin/trainer.py, icefall save_checkpoint)
+    """the trainer's checkpoint, {"model": state_dict, ...flattened params} (valle/bin/trainer.py, icefall
+    save_checkpoint), of the reference class initialised under torch.manual_seed(seed).  tests/golden/ref_layout.pt
+    holds the reference's state_dict layout and per-tensor fingerprints; the tensors are rebuilt by this package's
+    init, which must reproduce those fingerprints."""
+    from conftest import assert_checksums, build_model, load_golden
+    ref = load_golden("ref_layout.pt")[f"seed{seed}"]
+    src = build_model(dict(d_model=PARAMS["decoder_dim"], nhead=PARAMS["nhead"], num_layers=PARAMS["num_decoder_layers"],
+                           prefix_mode=1, num_quantizers=8), seed)
+    assert_checksums(src, ref["checksums"])
     ckpt = dict(PARAMS)
-    ckpt["model"] = rm.state_dict()
+    ckpt["model"] = src.state_dict()
     buf = io.BytesIO()
     torch.save(ckpt, buf)
     buf.seek(0)
-    return rm, torch.load(buf, map_location="cpu", weights_only=False)
+    return ref, torch.load(buf, map_location="cpu", weights_only=False)
 
 
 def test_infer_py_checkpoint_loading_from_a_reference_saved_checkpoint():
     """valle/bin/infer.py:126-144: checkpoint = torch.load(...); model = get_model(AttributeDict(checkpoint));
     missing, unexpected = model.load_state_dict(checkpoint["model"], strict=True); assert not missing"""
+    from conftest import assert_checksums
     from valle.models import get_model
     from valle.utils import AttributeDict
-    rm, ckpt = _reference_checkpoint(seed=123)
+    ref, ckpt = _reference_checkpoint(seed=123)
+    torch.manual_seed(999)            # a different init, fully overwritten by the load
     model = get_model(AttributeDict(ckpt))
     missing, unexpected = model.load_state_dict(ckpt["model"], strict=True)
     assert not missing and not unexpected
-    ours, theirs = model.state_dict(), rm.state_dict()
-    assert list(ours.keys()) == list(theirs.keys())
-    for k in ours:
-        assert ours[k].shape == theirs[k].shape and torch.equal(ours[k], theirs[k]), k
+    # the reference's keys in its order, shapes, dtypes and values
+    assert {k: (tuple(v.shape), v.dtype) for k, v in model.state_dict().items()} == ref["tensors"]
+    assert_checksums(model, ref["checksums"])
     # tied weights survive the load (valle.py:261-271)
     for j in range(6):
         assert model.nar_predict_layers[j].weight is model.nar_audio_embeddings[j + 2].weight
-    # and the other way round: a checkpoint saved by this class loads into the reference class
-    rm.load_state_dict(model.state_dict(), strict=True)
+    # and the other way round: a checkpoint saved by this class loads into the reference class, whose strict load
+    # needs exactly the key set and shapes checked above
+    assert [n for n, _ in model.named_parameters()] == ref["parameters"]
+    assert [n for n, _ in model.named_buffers()] == ref["buffers"]
 
 
 @pytest.mark.gpu

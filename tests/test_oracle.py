@@ -1,5 +1,5 @@
-"""CPU tests of the oracle: (1) against the reference itself when /root/reference is mounted
-(build container), (2) against the committed reference-generated golden fixtures (always)."""
+"""CPU tests of the oracle against outputs of the reference itself, stored under tests/golden/ by
+oracle/gen_golden.py."""
 import random
 
 import pytest
@@ -7,9 +7,6 @@ import torch
 
 from conftest import assert_checksums, build_model, load_golden
 from oracle import valle_oracle as O
-from oracle.ref_loader import load_reference, reference_available
-
-needs_ref = pytest.mark.skipif(not reference_available(), reason="/root/reference not mounted")
 
 
 def _sd(m):
@@ -74,63 +71,45 @@ def test_sampling_restatement_greedy_is_argmax():
     assert torch.equal(O.top_k_top_p_filtering(logits.clone(), top_k=-100), logits)
 
 
-@needs_ref
 @pytest.mark.parametrize("pm", [0, 1])
 def test_oracle_vs_reference_inference_and_forward(pm):
-    ref = load_reference()
-    torch.manual_seed(0)
-    m = ref.VALLE(256, 4, 2, norm_first=True, add_prenet=False, prefix_mode=pm, share_embedding=True,
-                  nar_scale_factor=1.0, prepend_bos=False, num_quantizers=8).eval()
+    """greedy and continual codes, top-k sampled codes at a fixed torch seed (the oracle consumes torch's RNG as the
+    reference does) and a training loss, against the reference's own outputs on the same weights and inputs"""
+    g = load_golden("ref_oracle.pt")[f"pm{pm}"]
+    m = build_model(g["config"], g["weight_seed"])
+    assert_checksums(m, g["checksums"])
     sd = _sd(m)
-    cfg = O.OracleConfig(256, 4, 2, pm, 8)
-    g = torch.Generator().manual_seed(21)
-    x = torch.randint(3, 100, (1, 7), generator=g)
-    y = torch.randint(0, 1024, (1, 15, 8), generator=g)
-    xl = torch.tensor([7], dtype=torch.int32)
+    cfg = O.OracleConfig(**g["config"])
+    x, y = g["x"], g["y"]
+    xl = torch.tensor([x.shape[1]], dtype=torch.int32)
     with torch.no_grad():
-        assert torch.equal(m.inference(x, xl, y, None, top_k=1), O.inference(sd, cfg, x, xl, y, None, top_k=1))
-        assert torch.equal(m.continual(x, xl, y), O.continual(sd, cfg, x, xl, y))
-    # sampled decoding consumes torch's RNG identically
-    with torch.no_grad():
+        assert torch.equal(O.inference(sd, cfg, x, xl, y, None, top_k=1), g["codes"].long())
+        assert torch.equal(O.continual(sd, cfg, x, xl, y), g["continual"].long())
         torch.manual_seed(3)
-        a = m.inference(x, xl, y, None, top_k=5, temperature=0.9)
-        torch.manual_seed(3)
-        b = O.inference(sd, cfg, x, xl, y, None, top_k=5, temperature=0.9)
-    assert torch.equal(a, b)
-    N = 3
-    xx = torch.randint(3, 100, (N, 9), generator=g)
-    xls = torch.tensor([9, 7, 5], dtype=torch.int32)
-    yy = torch.randint(0, 1024, (N, 40, 8), generator=g)
-    yls = torch.tensor([40, 33, 28], dtype=torch.int32)
-    m.rng = random.Random(0)
+        assert torch.equal(O.inference(sd, cfg, x, xl, y, None, top_k=5, temperature=0.9), g["sampled"].long())
+    fw = g["forward"]
+    xx, xls, yy, yls = fw["x"], fw["x_lens"], fw["y"].long(), fw["y_lens"]
+    # the NAR stage and the prompt prefix the reference drew with m.rng = random.Random(0) and torch.manual_seed(5)
     ns = random.Random(0).choices(list(range(1, 8)), weights=[1 / 7] * 7, k=1)[0]
-    torch.manual_seed(5)
-    with torch.no_grad():
-        (_, _), loss, _ = m(xx, xls, yy, yls)
     torch.manual_seed(5)
     int_low = (0.25 * yls.min()).type(torch.int64).item()
     pl = min(torch.randint(int_low, int_low * 2, size=()).item(), 225) if pm == 1 else 0
     with torch.no_grad():
         l2, _ = O.forward_train(sd, cfg, xx, xls, yy, yls, ns, pl)
-    assert abs(float(loss) - float(l2)) <= 1e-5 * abs(float(loss))
+    loss = float(fw["loss"])
+    assert abs(loss - float(l2)) <= 1e-5 * abs(loss)
 
 
-@needs_ref
 @pytest.mark.parametrize("prenet", [False, True])
 def test_model_mirror_matches_reference_checkpoint_layout(prenet):
-    """valle_b200.models.VALLE: same state_dict keys, shapes, init values and strict loading -- also with the
+    """valle_b200.models.VALLE: same state_dict keys, shapes, dtypes, init values and strict loading -- also with the
     pre-nets of add_prenet=True (Conv1d / BatchNorm1d / Linear containers at the reference's Sequential indices)."""
-    ref = load_reference()
+    ref = load_golden("ref_layout.pt")[f"prenet{int(prenet)}"]
     cfg = dict(d_model=256, nhead=4, num_layers=2, prefix_mode=1, num_quantizers=8, add_prenet=prenet)
-    torch.manual_seed(0)
-    a = ref.VALLE(256, 4, 2, norm_first=True, add_prenet=prenet, prefix_mode=1, share_embedding=True,
-                  nar_scale_factor=1.0, prepend_bos=False, num_quantizers=8)
     b = build_model(cfg, 0)
-    sa, sb = a.state_dict(), b.state_dict()
-    assert list(sa.keys()) == list(sb.keys())
-    assert all(torch.equal(sa[k], sb[k]) for k in sa)
-    b.load_state_dict(sa, strict=True)
-    a.load_state_dict(sb, strict=True)
-    assert [n for n, _ in a.named_parameters()] == [n for n, _ in b.named_parameters()]
-    assert [n for n, _ in a.named_buffers()] == [n for n, _ in b.named_buffers()]
+    assert {k: (tuple(v.shape), v.dtype) for k, v in b.state_dict().items()} == ref["tensors"]
+    assert_checksums(b, ref["checksums"])   # same keys in the same order, same init values
+    b.load_state_dict({k: torch.zeros(s, dtype=dt) for k, (s, dt) in ref["tensors"].items()}, strict=True)
+    assert [n for n, _ in b.named_parameters()] == ref["parameters"]
+    assert [n for n, _ in b.named_buffers()] == ref["buffers"]
     assert (len(list(b.named_buffers())) == 0) == (not prenet)

@@ -322,17 +322,18 @@ def test_ln_fold_build_matches_its_definition():
 
 
 @pytest.mark.parametrize("name", ["tiny_batch.pt", "big_short.pt"])
-def test_folded_decode_chain_matches_the_unfolded_chain(name):
+def test_folded_decode_chain_matches_the_unfolded_chain(name, monkeypatch):
     """The bf16 decode step with the LayerNorms folded into the projections (6 launches per layer: fp32-fed
     projections carrying the rows' moments, residual stream assembled by bulk reductions) against the chain with the
     separate residual + LayerNorm launches on the same weights: per-step logits within 2e-2 (both round to bf16 at
-    different points), the same early greedy ids, and the folded chain is what the engine runs by default."""
+    different points) and the same early greedy ids.  The folded chain runs on request (VB_DECODE_FOLD=1)."""
     from valle_b200 import _lib as L
     lib = L.load()
     g = load_golden(name)
+    monkeypatch.setenv("VB_DECODE_FOLD", "1")
     m = _model(g, torch.bfloat16)
     eng = m.engine()
-    assert eng.ar_head_fold is not None, "the LayerNorm-folded chain must be on by default in bf16"
+    assert eng.ar_head_fold is not None, "VB_DECODE_FOLD=1 must turn the LayerNorm-folded chain on in bf16"
     if "utts" in g:
         texts = [u["x"][0] for u in g["utts"]] * 3
         prompts = [u["y"][0] for u in g["utts"]] * 3

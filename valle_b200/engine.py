@@ -142,8 +142,10 @@ class ValleEngine:
         self.last_packed: Optional[torch.Tensor] = None
         #: rows of one tensor-core decode group (gemm_decode.cu: one UMMA N tile); larger bf16 batches are split
         self.max_tc_batch = 64
-        #: bf16 decode steps run the LayerNorm-folded chain (6 launches per layer instead of 8)
-        self.use_decode_fold = os.environ.get("VB_DECODE_FOLD", "1") != "0"
+        #: bf16 decode steps run the LayerNorm-folded chain (6 launches per layer instead of 8) only on request
+        #: (VB_DECODE_FOLD=1): it adds the split-K partials of the residual updates in arrival order, so a greedy decode
+        #: can differ between two runs after a near-tie; the default chain adds them in fixed order and is reproducible
+        self.use_decode_fold = os.environ.get("VB_DECODE_FOLD", "0") != "0"
         #: greedy decode steps captured per CUDA graph (one replay per group; the stop flags are polled every `poll` steps)
         self.steps_per_graph = 8
         self.replayed_launches = 0   # kernels executed through CUDA-graph replays
