@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define VB_ABI_VERSION 4
+#define VB_ABI_VERSION 5
 
 enum vb_status { VB_OK = 0, VB_ERR_ARG = 1, VB_ERR_CUDA = 2, VB_ERR_UNSUPPORTED = 3 };
 /* storage type of the big matrices / activations.  Accumulation is always fp32. */
@@ -293,6 +293,10 @@ typedef struct vb_ar_state {
   int64_t cache_layer_stride, cache_seq_stride; /* in elements */
   int32_t cache_cap;
   int32_t n_active_out_unused;
+  /* seeded sampling on the device (vb_ar_head.greedy == 2), [B] each; NULL otherwise */
+  const uint64_t *seed;       /* per-utterance seed s_b */
+  const int32_t *top_k;       /* per-utterance top_k (<= 0: no filter) */
+  const float *temperature;   /* per-utterance temperature (finite, > 0) */
 } vb_ar_state;
 
 typedef struct vb_ar_head {
@@ -303,9 +307,23 @@ typedef struct vb_ar_head {
   const float *alpha;         /* ar_audio_position.alpha (device scalar) */
   const float *pe;            /* fp32 [pe_rows, d] sine table */
   int32_t pe_rows;
-  int32_t greedy;             /* 1: argmax + stop rule + append on device; 0: logits only */
+  int32_t greedy;             /* 1: argmax + stop rule + append on device; 0: logits only;
+                                 2: seeded sampling + stop rule + append on device (below) */
   vb_ln_fold fold;            /* final LayerNorm folded into predict_w (all-NULL: separate LayerNorm launch) */
 } vb_ar_head;
+
+/* Seeded sampling (greedy == 2; vb_ar_state.seed / top_k / temperature set; n_vocab <= 1280).  The draw of utterance b
+ * at decode step t = n_gen[b] depends only on its logits row, s_b = seed[b], t, top_k[b] and temperature[b] -- not on
+ * its batch slot, the batch size or any other row:
+ *   1. z_i = logits_i / T  (IEEE fp32 division; valle.py:1297-1298 `logits / temperature`)
+ *   2. top_k > 0: k = min(top_k, n_vocab); keep every z_i >= (k-th largest z), ties with the k-th value included
+ *      (top_k_top_p_filtering, valle.py:1254-1260); top_k <= 0: keep all
+ *   3. Gumbel-max over the kept ids: h = mix64(s_b, t, i) >> 40 (24 bits; mix64 = the splitmix64 finaliser of the
+ *      dropout masks, z = s + t * 0x9E3779B97F4A7C15 + i * 0xD1342543DE82EF95 then xor-shift-multiply), u = (h + 0.5)
+ *      2^-24, e = -log(u) in fp32 (logf(u) for h < 2^23, else log1pf(-(2^24 - 1 - h + 0.5) 2^-24): both arguments are
+ *      exact), key_i = z_i - logf(e); sample = argmax key, lowest id on an exact tie.  This is a draw from
+ *      softmax(filtered z), as torch.multinomial(softmax(...), 1) draws.
+ *   4. stop rule unchanged (valle.py:1044-1048): argmax(logits) == eos, or sample == eos, or the cap. */
 
 /* bytes of scratch for vb_ar_head_step / vb_ar_decode_step.  The buffer must not be shared between
  * concurrently running streams. */

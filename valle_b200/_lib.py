@@ -12,7 +12,7 @@ from typing import Optional
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "lib", "libvalle_b200.so")
 
-ABI_VERSION = 4
+ABI_VERSION = 5
 VB_F32, VB_BF16 = 0, 1
 VB_EPI_NONE, VB_EPI_RELU, VB_EPI_RESIDUAL = 0, 1, 2
 VB_MASK_FULL, VB_MASK_VALLE_AR, VB_MASK_PADDED_AR, VB_MASK_PADDED, VB_MASK_DENSE = 0, 1, 2, 3, 4
@@ -44,7 +44,8 @@ class ArState(C.Structure):
                 ("n_gen", vp), ("finished", vp), ("tokens", vp), ("x_cur", vp), ("logits", vp),
                 ("kcache", vp), ("vcache", vp),
                 ("cache_layer_stride", C.c_int64), ("cache_seq_stride", C.c_int64),
-                ("cache_cap", C.c_int32), ("_unused", C.c_int32)]
+                ("cache_cap", C.c_int32), ("_unused", C.c_int32),
+                ("seed", vp), ("top_k", vp), ("temperature", vp)]
 
 
 class LnFold(C.Structure):

@@ -9,6 +9,16 @@ namespace vb {
 // a stateless Bernoulli mask keyed by (seed of the forward call, stream id of the site, element index), so the backward
 // pass regenerates the mask of the forward pass instead of storing it.  splitmix64 finaliser; keep <=> hash >= thresh
 // with thresh = p * 2^32.  tests/test_backward_gpu.py holds the same function in numpy.
+// The seeded AR sampler (sample.cu) draws its uniforms from the same hash, keyed by (utterance seed, decode step, id).
+__host__ __device__ __forceinline__ uint64_t mix64(uint64_t seed, uint64_t stream, uint64_t idx) {
+  uint64_t z = seed + stream * 0x9E3779B97F4A7C15ull + idx * 0xD1342543DE82EF95ull;
+  z ^= z >> 30;
+  z *= 0xBF58476D1CE4E5B9ull;
+  z ^= z >> 27;
+  z *= 0x94D049BB133111EBull;
+  z ^= z >> 31;
+  return z;
+}
 struct DropCfg {
   uint64_t seed;
   uint32_t stream;     // site id: (layer << 2) | {0 attention probabilities, 1 after out-proj, 2 FFN hidden, 3 after FFN}
@@ -17,13 +27,7 @@ struct DropCfg {
   int64_t lmax;        // attention only: index = ((b * H + h) * lmax + q) * lmax + k
 };
 __host__ __device__ __forceinline__ bool drop_keep(const DropCfg &c, uint64_t idx) {
-  uint64_t z = c.seed + (uint64_t)c.stream * 0x9E3779B97F4A7C15ull + idx * 0xD1342543DE82EF95ull;
-  z ^= z >> 30;
-  z *= 0xBF58476D1CE4E5B9ull;
-  z ^= z >> 27;
-  z *= 0x94D049BB133111EBull;
-  z ^= z >> 31;
-  return (uint32_t)(z >> 32) >= c.thresh;
+  return (uint32_t)(mix64(c.seed, c.stream, idx) >> 32) >= c.thresh;
 }
 inline DropCfg make_drop(float p, uint64_t seed, uint32_t stream, int64_t lmax = 0) {
   DropCfg c{};

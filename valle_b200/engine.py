@@ -18,6 +18,7 @@ libvalle_b200.so.  There is no CPU fallback.
 """
 from __future__ import annotations
 
+import math
 import os
 
 import ctypes as C
@@ -56,6 +57,31 @@ def _check_ids(tensors, hi: int, what: str):
                 raise IndexError(f"index out of range in self: {what} id {lo_v if lo_v < 0 else hi_v} not in [0, {hi})")
 
 
+def _per_utterance(v) -> bool:
+    """a list / tuple / 1-d array of per-utterance values rather than one scalar"""
+    return isinstance(v, (list, tuple)) or (isinstance(v, (torch.Tensor, np.ndarray)) and v.ndim > 0)
+
+
+def _sampling_params(B: int, seeds, top_k, temperature):
+    """validated per-utterance (seeds, top_k, temperature) lists of a seeded generate(); None without seeds"""
+    if seeds is None:
+        if _per_utterance(top_k) or _per_utterance(temperature):
+            raise ValueError("per-utterance top_k / temperature need per-utterance seeds")
+        return None
+    seeds = [int(s) for s in seeds]
+    if len(seeds) != B:
+        raise ValueError(f"{len(seeds)} seeds for {B} utterances")
+    if any(s < 0 or s >= 1 << 64 for s in seeds):
+        raise ValueError("a seed is not in [0, 2**64)")
+    ks = [int(k) for k in top_k] if _per_utterance(top_k) else [int(top_k)] * B
+    ts = [float(t) for t in temperature] if _per_utterance(temperature) else [float(temperature)] * B
+    if len(ks) != B or len(ts) != B:
+        raise ValueError(f"per-utterance top_k / temperature must have {B} entries")
+    if any(not math.isfinite(t) or t <= 0.0 for t in ts):
+        raise ValueError("temperature must be finite and > 0")
+    return seeds, ks, ts
+
+
 @dataclass
 class EngineStats:
     """CUDA-event timings (ms) of the phases of the last generate() call and the number of decode steps"""
@@ -83,6 +109,10 @@ class _ArBuffers:
         self.x_cur = torch.zeros((B, d), dtype=torch.float32, device=dev)
         self.ldl = (eng.n_vocab + 3) // 4 * 4
         self.logits = torch.zeros((B, self.ldl), dtype=torch.float32, device=dev)
+        # seeded sampling on the device (generate(seeds=...)): the uint64 seeds as int64 bit patterns, top_k, temperature
+        self.seed = torch.zeros(B, dtype=torch.int64, device=dev)
+        self.top_k = torch.zeros(B, **i32)
+        self.temperature = torch.ones(B, dtype=torch.float32, device=dev)
         self.kcache = torch.zeros((nd.n_layer, B, nd.H, cap, 64), dtype=eng.dtype, device=dev)
         self.vcache = torch.zeros_like(self.kcache)
         st = L.ArState()
@@ -92,6 +122,7 @@ class _ArBuffers:
         st.x_cur, st.logits = self.x_cur.data_ptr(), self.logits.data_ptr()
         st.kcache, st.vcache = self.kcache.data_ptr(), self.vcache.data_ptr()
         st.cache_layer_stride, st.cache_seq_stride, st.cache_cap = self.kcache.stride(0), self.kcache.stride(1), cap
+        st.seed, st.top_k, st.temperature = self.seed.data_ptr(), self.top_k.data_ptr(), self.temperature.data_ptr()
         self.st = st
         nbytes = eng.lib.vb_ar_step_workspace(C.byref(nd.desc), B, cap)
         self.ws = torch.zeros(nbytes, dtype=torch.uint8, device=dev)
@@ -146,7 +177,8 @@ class ValleEngine:
         #: (VB_DECODE_FOLD=1): it adds the split-K partials of the residual updates in arrival order, so a greedy decode
         #: can differ between two runs after a near-tie; the default chain adds them in fixed order and is reproducible
         self.use_decode_fold = os.environ.get("VB_DECODE_FOLD", "0") != "0"
-        #: greedy decode steps captured per CUDA graph (one replay per group; the stop flags are polled every `poll` steps)
+        #: decode steps captured per CUDA graph, greedy or seeded sampling (one replay per group; the stop flags are
+        #: polled every `poll` steps)
         self.steps_per_graph = 8
         self.replayed_launches = 0   # kernels executed through CUDA-graph replays
         self.captured_launches = 0   # kernels recorded at capture time (counted by the library, not run)
@@ -245,7 +277,7 @@ class ValleEngine:
             self._ada_cache = [self.nar.ada_table(e.weight) for e in self.model.nar_stage_embeddings]
         return self._ada_cache
 
-    def _head(self, pe: torch.Tensor, greedy: bool) -> L.ArHead:
+    def _head(self, pe: torch.Tensor, mode: int) -> L.ArHead:
         m = self.model
         h = L.ArHead()
         h.predict_w = self.ar_predict_w.data_ptr()
@@ -253,7 +285,7 @@ class ValleEngine:
         h.audio_emb = self.ar_audio_table.data_ptr()      # the embedding table, or pre-net(embedding) (add_prenet)
         h.alpha = m.ar_audio_position.alpha.detach().data_ptr()
         h.pe, h.pe_rows = pe.data_ptr(), pe.shape[0]
-        h.greedy = int(greedy)
+        h.greedy = mode          # 0 logits only, 1 argmax, 2 seeded sampling (vb_ar_head.greedy)
         if self.ar_head_fold is not None:
             h.fold = self.ar_head_fold
         return h
@@ -272,12 +304,21 @@ class ValleEngine:
     @torch.no_grad()
     @_on_device
     def generate(self, texts: Sequence[torch.Tensor], prompts: Sequence[torch.Tensor],
-                 enroll_lens: Optional[Sequence[int]] = None, top_k: int = 1, temperature: float = 1.0,
+                 enroll_lens: Optional[Sequence[int]] = None, top_k=1, temperature=1.0,
                  max_new_tokens: Optional[int] = None, poll: int = 32,
                  return_device: bool = False, trace: Optional[dict] = None,
-                 forced: Optional[Sequence[torch.Tensor]] = None) -> List[torch.Tensor]:
+                 forced: Optional[Sequence[torch.Tensor]] = None,
+                 seeds: Optional[Sequence[int]] = None) -> List[torch.Tensor]:
         """texts[b]: int64 [S_b] phoneme ids; prompts[b]: int64 [Tp_b, Q] codec ids (host or device).
         Returns codes[b]: int64 [Tgen_b, Q] -- per utterance exactly what VALLE.inference returns.
+
+        Sampling (valle.py:1040-1043): top_k == 1 decodes greedily.  Otherwise, without `seeds`, the ids are drawn with
+        torch's generator as the reference draws them (one multinomial over the batch per step, or per utterance on the
+        host with `sample_on_host`), so a draw depends on the batch it is part of.  With `seeds` (one int in [0, 2**64)
+        per utterance) the draw runs in the sampler kernel inside the graph-replayed decode step and depends only on the
+        utterance's logits, seed, step, top_k and temperature (include/valle_b200.h): the same utterance and seed give
+        the same codes alone, in any batch slot or group, on any rank.  top_k and temperature may then be one value per
+        utterance.
 
         Test hooks: `trace` collects AR logits (trace["steps"] = set of iterations or "all") and, with
         trace["nar"] = True, the NAR logits / argmax of every stage; `forced[b]` = int64 [T_b, Q] codes the decode is
@@ -287,6 +328,11 @@ class ValleEngine:
         m, dev, d, Q = self.model, self.device, self.d, self.Q
         B = len(texts)
         assert B == len(prompts) and B >= 1
+        sampling = _sampling_params(B, seeds, top_k, temperature)
+        if sampling is not None and self.sample_on_host:
+            raise ValueError("seeds draw on the device: they cannot be combined with sample_on_host=True")
+        if sampling is not None and forced is not None:
+            raise ValueError("seeds cannot be combined with forced ids")
         if B > self.max_tc_batch and self.dtype == torch.bfloat16 and trace is None and forced is None:
             # the tensor-core decode projections take up to 64 rows (one UMMA N tile): a larger batch is decoded as
             # consecutive groups of <= 64 utterances instead of falling onto the CUDA-core GEMV path
@@ -295,8 +341,12 @@ class ValleEngine:
             packed = []
             for b0 in range(0, B, self.max_tc_batch):
                 b1 = min(B, b0 + self.max_tc_batch)
+                if sampling is None:
+                    k_g, t_g, s_g = top_k, temperature, None
+                else:  # every utterance keeps its own seed and parameters
+                    s_g, k_g, t_g = (v[b0:b1] for v in sampling)
                 outs += self.generate(texts[b0:b1], prompts[b0:b1], None if enroll_lens is None else enroll_lens[b0:b1],
-                                      top_k, temperature, max_new_tokens, poll, return_device, None, None)
+                                      k_g, t_g, max_new_tokens, poll, return_device, None, None, seeds=s_g)
                 stats.ar_steps += self.stats.ar_steps
                 stats.ar_ms += self.stats.ar_ms
                 stats.prefill_ms += self.stats.prefill_ms
@@ -319,7 +369,9 @@ class ValleEngine:
             cap_new = [min(c, max_new_tokens - 1) for c in cap_new]
         tok_stride = (max(cap_new) + 2 + 7) // 8 * 8
         cap = (max(S[b] + Tp[b] + cap_new[b] + 2 for b in range(B)) + 63) // 64 * 64
-        greedy = top_k == 1 and forced is None
+        greedy = sampling is None and top_k == 1 and forced is None
+        seeded = sampling is not None
+        on_device = greedy or seeded  # the sampler kernel picks the id: decode steps replay as CUDA graphs
         forced_steps = None
         if forced is not None:  # [steps, B] first-codebook ids, EOS once an utterance's forced ids run out
             n_f = max(int(f.shape[0]) for f in forced) + 1
@@ -367,6 +419,11 @@ class ValleEngine:
         buf.max_new.copy_(capn_d)
         buf.n_gen.zero_()
         buf.finished.zero_()
+        if seeded:
+            s_l, k_l, t_l = sampling
+            buf.seed.copy_(torch.tensor([s - (1 << 64) if s >= 1 << 63 else s for s in s_l], dtype=torch.int64))
+            buf.top_k.copy_(torch.tensor(k_l, dtype=torch.int32))
+            buf.temperature.copy_(torch.tensor(t_l, dtype=torch.float32))
         pe_t = self._pe(m.ar_text_position, max(S))
         pe_a = self._pe(m.ar_audio_position, max(Tp) + max(cap_new) + 2)
         x = torch.empty((M, d), dtype=torch.float32, device=dev)
@@ -378,7 +435,7 @@ class ValleEngine:
             self._embed_pe(prm_all, Q, self.ar_audio_table, pe_a, m.ar_audio_position.alpha, sum(Tp), x, arow_d, apos_d)
         self.ar.forward(x, cu_d, B, max(seq_len), L.VB_MASK_VALLE_AR, S_d, None, buf.kcache, buf.vcache, cap)
         h_last = ops.gather_rows(x, last_d)
-        head = self._head(pe_a, greedy)
+        head = self._head(pe_a, 2 if seeded else int(greedy))
         self._head_ref = head
         L.check(self.lib.vb_ar_head_step(self.ar.handle, C.byref(head), h_last.data_ptr(), C.byref(buf.st),
                                          buf.ws.data_ptr(), buf.ws.numel(), L.stream_ptr()), "vb_ar_head_step")
@@ -392,7 +449,7 @@ class ValleEngine:
             poll = 1
         if forced_steps is not None:
             poll = 1
-        if not greedy:
+        if not on_device:
             self._sample_push(buf, head, top_k, temperature, None if forced_steps is None else forced_steps[0])
         if any(t.is_cuda for t in list(texts) + list(prompts)):
             ops.check_oob(dev)  # ids that were already on the device are range-checked by the embedding kernels
@@ -403,7 +460,7 @@ class ValleEngine:
         steps = 0
         while steps < max_steps:
             n = min(poll, max_steps - steps)
-            if greedy and self.use_cuda_graph:
+            if on_device and self.use_cuda_graph:
                 # whole groups of `steps_per_graph` decode steps as one graph replay (no launch gap between the
                 # steps of a group), the remainder one step at a time
                 done = 0
@@ -416,7 +473,7 @@ class ValleEngine:
                     fs = None
                     if forced_steps is not None:
                         fs = forced_steps[min(steps + 1, forced_steps.shape[0] - 1)]
-                    self._decode_step(buf, head, greedy, top_k, temperature, fs)
+                    self._decode_step(buf, head, on_device, top_k, temperature, fs)
             steps += n
             if trace is not None and want(steps):  # poll == 1 here: the logits row of iteration `steps`
                 trace["ar_logits"][steps] = buf.logits[:, : self.n_vocab].clone()
@@ -503,10 +560,11 @@ class ValleEngine:
             tmp = self._text_prenet(tmp, prenet[1], prenet[0])
         ops.add_pe(tmp, pe, alpha.detach(), x, n, positions=pos, out_rows=rows)
 
-    def _decode_step(self, buf: _ArBuffers, head: L.ArHead, greedy: bool, top_k: int, temperature: float,
+    def _decode_step(self, buf: _ArBuffers, head: L.ArHead, on_device: bool, top_k: int, temperature: float,
                      forced_step: Optional[torch.Tensor] = None):
-        if greedy and self.use_cuda_graph:
-            key = (head.pe, head.predict_w, head.audio_emb)
+        """one decode step; on_device: the sampler kernel picks the id (greedy or seeded), else _sample_push draws it"""
+        if on_device and self.use_cuda_graph:
+            key = (head.pe, head.predict_w, head.audio_emb, head.greedy)
             if buf.graph is not None and buf.graph_key != key:
                 buf.graph = None
             if buf.graph is None:
@@ -526,12 +584,13 @@ class ValleEngine:
             self.replayed_launches += buf.graph_kernels
             return
         self._launch_step(buf, head)
-        if not greedy:
+        if not on_device:
             self._sample_push(buf, head, top_k, temperature, forced_step)
 
     def _replay_steps(self, buf: _ArBuffers, head: L.ArHead, k: int):
-        """k greedy decode steps as ONE CUDA graph (captured on first use per (buffer, head tables, k))"""
-        key = (head.pe, head.predict_w, head.audio_emb, k)
+        """k decode steps (greedy or seeded sampling) as ONE CUDA graph (captured on first use per (buffer, head tables,
+        head mode, k)); the seeds and sampling parameters are read from the buffer's device arrays at every replay"""
+        key = (head.pe, head.predict_w, head.audio_emb, head.greedy, k)
         graphs = buf.__dict__.setdefault("graphs", {})
         ent = graphs.get(key)
         if ent is None:

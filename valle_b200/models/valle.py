@@ -211,9 +211,12 @@ class VALLE(nn.Module):
     @torch.no_grad()
     def inference(self, x: torch.Tensor, x_lens: torch.Tensor, y: torch.Tensor,
                   enroll_x_lens: Optional[torch.Tensor] = None, top_k: int = -100,
-                  temperature: float = 1.0, max_new_tokens: Optional[int] = None) -> torch.Tensor:
+                  temperature: float = 1.0, max_new_tokens: Optional[int] = None,
+                  seed: Optional[int] = None) -> torch.Tensor:
         """x: (1, S) phoneme ids, x_lens: (1,), y: (1, T, 8) acoustic prompt.
-        Returns the predicted audio code matrix (1, T', 8) -- same contract as the reference."""
+        Returns the predicted audio code matrix (1, T', 8) -- same contract as the reference.
+        seed (engine feature, int in [0, 2**64)): draw on the device keyed by this seed instead of torch's generator, so
+        the same call reproduces the same codes, alone or inside any inference_batch (ValleEngine.generate)."""
         assert x.ndim == 2, x.shape
         assert x_lens.ndim == 1, x_lens.shape
         assert y.ndim == 3, y.shape
@@ -223,20 +226,23 @@ class VALLE(nn.Module):
         enroll = [int(enroll_x_lens.max())] if (self.prefix_mode in (2, 4) and enroll_x_lens is not None) else None
         out = self.engine().generate([x[0, :S]], [y[0]], enroll_lens=enroll, top_k=top_k,
                                      temperature=temperature, max_new_tokens=max_new_tokens,
-                                     return_device=True)
+                                     return_device=True, seeds=None if seed is None else [seed])
         return out[0].unsqueeze(0).to(y.device)
 
     @torch.no_grad()
     def inference_batch(self, texts: Sequence[torch.Tensor], prompts: Sequence[torch.Tensor],
                         enroll_lens: Optional[Sequence[int]] = None, top_k: int = 1,
                         temperature: float = 1.0, max_new_tokens: Optional[int] = None,
-                        dtype: Optional[torch.dtype] = None, return_device: bool = False) -> List[torch.Tensor]:
+                        dtype: Optional[torch.dtype] = None, return_device: bool = False,
+                        seeds: Optional[Sequence[int]] = None) -> List[torch.Tensor]:
         """Engine feature (the reference asserts batch 1, valle.py:989): B independent utterances
         decoded together; result[b] equals `inference()` on utterance b alone.  Codes come back on the host, or
-        (return_device=True) stay on the GPU, e.g. for the data-parallel gather of valle_b200.dist."""
+        (return_device=True) stay on the GPU, e.g. for the data-parallel gather of valle_b200.dist.
+        seeds: one int per utterance for seeded sampling on the device; top_k / temperature may then be per utterance
+        (ValleEngine.generate)."""
         return self.engine(dtype).generate(texts, prompts, enroll_lens=enroll_lens, top_k=top_k,
                                            temperature=temperature, max_new_tokens=max_new_tokens,
-                                           return_device=return_device)
+                                           return_device=return_device, seeds=seeds)
 
     @torch.no_grad()
     def continual(self, x: torch.Tensor, x_lens: torch.Tensor, y: torch.Tensor) -> torch.Tensor:
